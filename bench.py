@@ -12,7 +12,8 @@ BASELINE configs[1]: coinrun, distribution_mode=easy) with synthetic uniform-ran
   cpu_baseline  oracle/_ref (reference game logic compiled unmodified + restated Qt raster) on the
           host cores, bounded sample
 With --impl reference the reference's CPU implementation (oracle/_ref, all host threads) is timed
-instead and reported on the same metric/config.
+instead and reported on the same metric/config. --dump-outputs DIR saves what the last timed step
+returned, so that two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -30,6 +31,8 @@ sys.path.insert(0, ROOT)
 
 ALGO_BYTES_PER_ENV_STEP = 64 * 64 * 3  # SURVEY §8(d)
 METRIC = "env-steps/sec"
+CLOCK_WARM_ROUNDS = 20   # of 20 steps each, before the steady-state timed steps
+DUMP_BYTES = 64 << 20    # --dump-outputs: all files together
 
 
 def measured_peak_gbs():
@@ -244,6 +247,29 @@ def reset_fraction(env, actions, t0, steps):
     return float(acc.item()) / (steps * env.num)
 
 
+def dump_outputs(env, out_dir):
+    """Writes what observe() returned after the last timed step as float32 .npy files: rew.npy and
+    first.npy for every env, and rgb.npy for a fixed seeded sample of envs whose indices are in
+    rgb_envs.npy, sized so that the four files stay within DUMP_BYTES."""
+    import numpy as np
+    import torch
+
+    rew, ob, first = env.observe()
+    n = rew.shape[0]
+    per_frame = 64 * 64 * 3 * 4 + 8   # float32 frame + its float64 index
+    room = DUMP_BYTES - 8 * n - 4 * 4096   # rew, first and the .npy headers
+    if room < per_frame:
+        raise SystemExit(f"--dump-outputs: {n} envs do not fit in {DUMP_BYTES} bytes")
+    k = min(n, room // per_frame)
+    envs = np.arange(n) if k == n else np.sort(np.random.RandomState(0).choice(n, k, replace=False))
+    rgb = ob["rgb"][torch.as_tensor(envs, device=ob["rgb"].device)]
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "rew.npy"), rew.float().cpu().numpy())
+    np.save(os.path.join(out_dir, "first.npy"), first.float().cpu().numpy())
+    np.save(os.path.join(out_dir, "rgb.npy"), rgb.float().cpu().numpy())
+    np.save(os.path.join(out_dir, "rgb_envs.npy"), envs.astype(np.float64))
+
+
 def max_over_ranks(x, dist, dev):
     import torch
 
@@ -312,10 +338,11 @@ def run_ours(args):
     # ---- steady state (the headline)
     sampler = ClockSampler(torch.cuda.current_device())
     sampler.start()
-    # the timed region can be as short as 50 ms: give nvidia-smi a second of the very same load first, so
-    # that the samples (taken every 25 ms until the timed region ends) describe the clocks it ran at
-    t_s = time.perf_counter()
-    while time.perf_counter() - t_s < 1.0:
+    # the timed region can be as short as 50 ms: give nvidia-smi the very same load first, so that the
+    # samples (taken every 25 ms until the timed region ends) describe the clocks it ran at. A fixed
+    # number of steps (about a second of the default workload on a B200), not a fixed time, so that
+    # the timed steps start from the same env state on every run.
+    for _ in range(CLOCK_WARM_ROUNDS):
         for t in range(20):
             env.act(actions[(steps_done + t) % T])
             env.observe()
@@ -324,6 +351,8 @@ def run_ours(args):
     elapsed_ms = max_over_ranks(timed_rollout(env, actions, steps_done, K, barrier, gather=args.gather, dist=dist), dist, dev)
     launches = env.kernel_launches() - launches0
     clocks = sampler.stop()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(env, args.dump_outputs)
     steps_done += K
     value = n * world * K / (elapsed_ms / 1000.0)
     value_cold = n * world * K / (cold_ms / 1000.0)
@@ -443,7 +472,11 @@ def run_ours(args):
         except Exception:
             traffic = None
     cpu = None
-    if not args.no_cpu_baseline:
+    from oracle.ref_env import REF_LIB
+
+    if not os.path.exists(REF_LIB):
+        cpu = {"value": None, "note": "not measured: oracle/_ref (built from the reference tree) is absent"}
+    elif not args.no_cpu_baseline:
         rate, detail = cpu_reference_rate(args.game, args.mode, budget_s=args.cpu_budget)
         cpu = {"value": rate, "unit": "env-steps/s", "cores": detail["cores"], "kind": "reference", "host": host_cpu_info(),
                "sample": detail["sample"] + "; reference game logic compiled unmodified + Qt raster restated on CPU"}
@@ -502,7 +535,13 @@ def main():
     ap.add_argument("--nccl-gather", action="store_true", help="keep the plain NCCL gather (no peer writes) for the gather measurements")
     ap.add_argument("--gather", action="store_true",
                     help="BASELINE configs[4] variant: NCCL-gather every step's rgb shard to rank 0 inside the timed region")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the observe() outputs of the last steady-state timed step to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
     if args.game == "all16":  # BASELINE configs[4]: env n plays game n % 16
         args.game = ALL16
     if args.warmup < 3 and args.impl == "ours":

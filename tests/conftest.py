@@ -30,9 +30,7 @@ def asset_pack():
     from procgen_b200 import assets
 
     if not os.path.exists(assets.DEFAULT_PACK):
-        if not os.path.isdir(assets.REFERENCE_ROOT):
-            pytest.skip("asset pack not built and reference tree absent")
-        assets.build_pack()
+        assets.build_pack_from_images()
     return assets.DEFAULT_PACK
 
 
@@ -48,8 +46,7 @@ def hostsim_lib(asset_pack):
 def product_lib():
     from procgen_b200 import build as B
 
-    # in the dev container (reference tree present) keep the in-tree library in step with the
-    # sources; on the GPU box use the library that travelled with the snapshot
-    if not os.path.exists(B.LIB_PATH) or (os.path.isdir("/root/reference") and B.needs_build()):
+    # never test a library older than the sources it was built from
+    if B.needs_build():
         B.build_library()
     return B.LIB_PATH
