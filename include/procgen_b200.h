@@ -210,6 +210,13 @@ LIBENV_API int pgb200_consumer_slot(libenv_env *handle);
  * header pgb200_debug_read_env returns; -1 in the product build. */
 LIBENV_API int pgb200_debug_phase_offset(void);
 
+/* Host debug build only: which path of the render kernel's gather each of the 64 x 64 pixels of env's
+ * last frame takes (0 tile cell, opaque texel | 1 tile cell, texel not opaque or empty cell | 2 overlap
+ * strip of two cell columns / rows | 3 solid-colour cell | 4 other general cell | 5 no cell), bit 7 set
+ * where the box of an entity or overlay blit covers the pixel; out = 4096 bytes, row-major. Returns 0,
+ * -1 in the product build. */
+LIBENV_API int pgb200_debug_pixel_classes(libenv_env *handle, int env, uint8_t *out);
+
 /* Introspection: shared memory of one render CTA (the per-game frame) and the number of render CTAs
  * per SM the render kernel of `game` is compiled for. Returns -1 for an unknown game. */
 LIBENV_API int pgb200_frame_info(const char *game, int *frame_bytes, int *ctas_per_sm);

@@ -211,13 +211,13 @@ template <class Frame>
 PG_HD void env_stage_tiles_serial(const KParams &p, Frame &f) {
     const int nj = f.n_tjobs < MAX_TILE_JOBS ? f.n_tjobs : MAX_TILE_JOBS;
     for (int j = 0; j < nj; j++)
-        for (int w = 0; w < (int)f.tjob_words[j]; w++) f.arena[f.tjob_dst[j] + w] = p.tiles.texels[f.tjob_src[j] + w];
+        for (int w = 0; w < (int)f.tjob[j].words; w++) f.arena[f.tjob[j].dst + w] = p.tiles.texels[f.tjob[j].src + w];
 }
 
 // Compose the rows row_first, row_first + row_step, ... of the frame (`lane` of `nlanes` threads own them)
 template <class G, class Frame>
-PG_HD void env_render_compose(const KParams &p, Frame &f, int row_first, int row_step, int lane, int nlanes) {
-    Raster<G, Frame>::compose_rows(f, f.fb, row_first, row_step, lane, nlanes, p.atlas);
+PG_HD void env_render_compose(const KParams &p, Frame &f, int row_first, int row_step, int lane, int nlanes, uint32_t *dbg = nullptr) {
+    Raster<G, Frame>::compose_rows(f, f.fb, row_first, row_step, lane, nlanes, p.atlas, dbg);
 }
 
 // Fill one tile of the global table (TileTable): tile (slot, tw, th) = the texels an un-clipped

@@ -125,9 +125,8 @@ struct RenderTune {
 #else
     // 227 KiB usable per SM, 1 KiB reserved per resident CTA
     static constexpr int kFit = (int)((227 * 1024) / (kFrameBytes + 1024 + 16));
-    // measured (profiles/r02_ab_render_ctas.txt): the games that draw grid cells run best at 7 CTAs (72
-    // registers: at 64 the gather loop spills), the entity-only games at 8
-    static constexpr int kWant = G::DRAWS_GRID ? 7 : 8;
+    // 8 CTAs = 64 registers, which the gather fits without spilling (profiles/r03_ab_render_ctas.txt)
+    static constexpr int kWant = 8;
     static constexpr int kMinBlocks = kFit >= kWant ? kWant : (kFit >= 1 ? kFit : 1);
 #endif
 };
@@ -140,6 +139,9 @@ __device__ __forceinline__ void pg_mbar_init(unsigned long long *bar, unsigned c
 }
 __device__ __forceinline__ void pg_mbar_arrive_expect_tx(unsigned long long *bar, unsigned bytes) {
     asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(pg_smem_addr(bar)), "r"(bytes) : "memory");
+}
+__device__ __forceinline__ void pg_mbar_expect_tx(unsigned long long *bar, unsigned bytes) {
+    asm volatile("mbarrier.expect_tx.relaxed.cta.shared::cta.b64 [%0], %1;" ::"r"(pg_smem_addr(bar)), "r"(bytes) : "memory");
 }
 __device__ __forceinline__ void pg_mbar_wait(unsigned long long *bar, unsigned parity) {
     unsigned done = 0;
@@ -203,22 +205,35 @@ __global__ void __launch_bounds__(kRenderThreads, RenderTune<G, VIEW>::kMinBlock
     if (tid < 32) {
         // Everything the setup kernel prepared for this env — one bulk copy into the head of the frame —
         // and the pre-scaled tiles its cells need, one bulk copy each, all counted on one mbarrier phase.
-        const int nj = G::DRAWS_GRID ? (gs->n_tjobs < MAX_TILE_JOBS ? gs->n_tjobs : MAX_TILE_JOBS) : 0;
-        unsigned words = 0;
-        for (int j = tid; j < nj; j += 32) words += gs->tjob_words[j];
-        for (int d = 16; d > 0; d >>= 1) words += __shfl_xor_sync(0xffffffffu, words, d);
+        // The record's copy goes first: its bytes are expected without arriving, so the phase cannot
+        // complete before the tile bytes are expected too (by the arrival, after the job records are read).
         if (tid == 0) {
-            pg_mbar_arrive_expect_tx(&f.mbar, (unsigned)sizeof(Shared) + 4u * words);
+            pg_mbar_expect_tx(&f.mbar, (unsigned)sizeof(Shared));
             pg_bulk_load(static_cast<Shared *>(&f), static_cast<const Shared *>(gs), (unsigned)sizeof(Shared), &f.mbar);
         }
+        const int nj = G::DRAWS_GRID ? (gs->n_tjobs < MAX_TILE_JOBS ? gs->n_tjobs : MAX_TILE_JOBS) : 0;
+        TileJob job = {0u, 0, 0};
+        if (tid < nj)
+            job = gs->tjob[tid];
+        unsigned words = job.words;
+        for (int j = tid + 32; j < nj; j += 32) words += gs->tjob[j].words;
+        for (int d = 16; d > 0; d >>= 1) words += __shfl_xor_sync(0xffffffffu, words, d);
+        if (tid == 0)
+            pg_mbar_arrive_expect_tx(&f.mbar, 4u * words);
         __syncwarp();
-        for (int j = tid; j < nj; j += 32)
-            pg_bulk_load(f.arena + gs->tjob_dst[j], p.tiles.texels + gs->tjob_src[j], 4u * gs->tjob_words[j], &f.mbar);
+        if (tid < nj)
+            pg_bulk_load(f.arena + job.dst, p.tiles.texels + job.src, 4u * job.words, &f.mbar);
+        for (int j = tid + 32; j < nj; j += 32)
+            pg_bulk_load(f.arena + gs->tjob[j].dst, p.tiles.texels + gs->tjob[j].src, 4u * gs->tjob[j].words, &f.mbar);
     }
     pg_mbar_wait(&f.mbar, 0);
     PG_RENDER_PHASE(0);
     // warp w owns rows y = w (mod warps): gather and paint need no block barrier in between
+#ifdef PG_PHASE_TIMING
+    env_render_compose<G, Frame>(p, f, tid >> 5, kRenderThreads >> 5, tid & 31, 32, p.hdr[env].dbg_phase + 8);  // 8 gather, 9 paint
+#else
     env_render_compose<G, Frame>(p, f, tid >> 5, kRenderThreads >> 5, tid & 31, 32);
+#endif
     __syncthreads();
     PG_RENDER_PHASE(5);
     if (p.consumer != nullptr) {
@@ -302,6 +317,51 @@ void render_env_serial(const KParams &p, int env, Frame &f) {
     for (int w = 0; w < 4; w++) env_render_compose<G, Frame>(p, f, w, 4, 0, 1);  // the device's row ownership, one lane per owner
     uint32_t *out = reinterpret_cast<uint32_t *>(p.rgb + (size_t)env * (RES_W * RES_H * 3));
     for (int g = 0; g < RES_W * RES_H / 4; g++) Raster<G, Frame>::pack_quad(f.fb + 4 * g, out + 3 * g);
+}
+
+// Which path of the gather each pixel of env's last frame takes (PixelClass), bit 7 set where an entity or
+// overlay blit's box covers it. Host debug build only, where the frame record is host memory; the
+// census of tools/render_pixel_classes.py.
+enum PixelClass : uint8_t { PC_TILE_OPAQUE = 0, PC_TILE_UNDER = 1, PC_STRIP = 2, PC_GEN_SOLID = 3, PC_GEN_OTHER = 4, PC_NO_CELL = 5, PC_PAINTED = 0x80 };
+template <class G, int VIEW>
+int frame_pixel_classes(const KParams &p, int env, uint8_t *out) {
+#ifdef PG_HOSTSIM
+    using Setup = typename FrameFor<G, VIEW>::setup;
+    const Setup &f = *reinterpret_cast<const Setup *>(p.frame_setup + (size_t)env * p.frame_setup_stride);
+    const int nj = f.n_tjobs < MAX_TILE_JOBS ? f.n_tjobs : MAX_TILE_JOBS;
+    for (int py = 0; py < RES_H; py++)
+        for (int px = 0; px < RES_W; px++) {
+            uint8_t cls = PC_NO_CELL;
+            const uint32_t ci = G::DRAWS_GRID ? f.colinfo[px] : 0u, ri = G::DRAWS_GRID ? f.rowinfo[py] : 0u;
+            if ((ci & ri & CI_VALID) && !(ci & ri & CI_FAST)) {
+                cls = PC_STRIP;
+            } else if (ci & ri & CI_FAST) {
+                const uint32_t code = f.cellmap[(ci & CI_BASE_MASK) + (ri & CI_BASE_MASK)];
+                if (code & CELL_GENERAL) {
+                    cls = f.gen_blit((int)(code & 0x7fffu))->kind == BLIT_SOLID ? PC_GEN_SOLID : PC_GEN_OTHER;
+                } else {
+                    uint32_t texel = 0;
+                    if (code) {  // arena word -> the table word its staging job copies there
+                        const uint32_t a = code - 1 + ((ri >> CI_D_SHIFT) & 31u) * ((ci >> CI_TW_SHIFT) & 31u) + ((ci >> CI_D_SHIFT) & 31u);
+                        for (int j = 0; j < nj; j++)
+                            if (a >= f.tjob[j].dst && a < (uint32_t)f.tjob[j].dst + f.tjob[j].words)
+                                texel = p.tiles.texels[f.tjob[j].src + a - f.tjob[j].dst];
+                    }
+                    cls = texel >= 0xff000000u ? PC_TILE_OPAQUE : PC_TILE_UNDER;
+                }
+            }
+            for (int i = 0; i < f.n_ent + f.n_overlay; i++) {
+                const Blit &b = f.ents[i];
+                if ((uint32_t)(px - b.x1) < b.w && (uint32_t)(py - b.y1) < b.h)
+                    cls |= PC_PAINTED;
+            }
+            out[py * RES_W + px] = cls;
+        }
+    return 0;
+#else
+    (void)p; (void)env; (void)out;
+    return -1;
+#endif
 }
 
 struct LaunchCtx {
@@ -422,6 +482,7 @@ struct GameVTable {
     void (*init[2])(const KParams &, const LaunchCtx &);
     void (*step[2])(const KParams &, const LaunchCtx &);
     void (*observe_only[2])(const KParams &, const LaunchCtx &);
+    int (*pixel_classes[2])(const KParams &, int, uint8_t *);
 };
 
 template <class G, int VIEW>
@@ -438,6 +499,7 @@ void fill_view(GameVTable &vt, int slot) {
     vt.init[slot] = &launch_env_kernel<G, true, VIEW>;
     vt.step[slot] = &launch_env_kernel<G, false, VIEW>;
     vt.observe_only[slot] = &launch_observe_only<G, VIEW>;
+    vt.pixel_classes[slot] = &frame_pixel_classes<G, VIEW>;
 }
 
 template <class G>

@@ -96,6 +96,13 @@ constexpr int CI_D_SHIFT = 13;                   // 5 bits: px - col_p1 (py - ro
 constexpr int CI_TW_SHIFT = 18;                  // 5 bits, column only: row stride of its tiles (0: not tile-eligible)
 constexpr uint32_t CI_MULTI = 1u << 23;          // more than one cell column / row covers the pixel
 constexpr uint32_t CI_FAST = 1u << 24;           // exactly one does
+constexpr uint32_t CI_WIDE = 1u << 25;           // more than two do (colinfo_lo / rowinfo_lo do not describe them all)
+
+// one pre-scaled tile to stage: texel offset in the table, arena word offset, words (one 8-byte load)
+struct alignas(8) TileJob {
+    uint32_t src;
+    uint16_t dst, words;
+};
 
 // One frame's working set, in three parts:
 //   FrameSharedT  what the setup kernel (one warp per env) hands to the render kernel: camera, cell
@@ -127,8 +134,7 @@ struct alignas(16) FrameSharedT {
     RotBlit *rot;                   // this env's rotated-sprite / span records (global)
     Blit *ents;                     // this env's blit list (global): the painter reads it sequentially
     Blit *gen_spill;                // this env's general cell blits (global): solid-colour cells, clipped walks that differ, un-snapped targets
-    int32_t n_strip_cols;           // pixel columns where two cell columns overlap
-    int32_t spare;
+    int32_t spare[2];
     // geometry shared by all cells of a column / row (the cell rect is separable)
     double cell_w;                  // QRectF.width == height
     double spare_d;
@@ -142,14 +148,15 @@ struct alignas(16) FrameSharedT {
     alignas(4) uint8_t row_p2[kSpanBytes];
     uint8_t col_tw[MAX_CELLS_1D], row_th[MAX_CELLS_1D];  // snapped size if the column / row can use tiles, else 0
     uint8_t col_k0[MAX_CELLS_1D], row_k0[MAX_CELLS_1D];  // pixels the device edge cuts off the near side (tile offset of the first visible one)
-    uint8_t strip_cols[RES_W];
     uint8_t col_lo[RES_W], col_hi[RES_W];   // window-relative cell columns covering pixel column
     uint8_t row_lo[RES_H], row_hi[RES_H];
-    alignas(4) uint32_t colinfo[RES_W];
-    uint32_t rowinfo[RES_H];                  // CI_* words
+    alignas(16) uint32_t colinfo[RES_W];      // CI_* words of the cell column (row) covering the pixel; the later one in
+    alignas(16) uint32_t rowinfo[RES_H];      // draw order where two overlap (CI_MULTI)
+    alignas(16) uint32_t colinfo_lo[RES_W];   // CI_MULTI: the same for the earlier of the two (else = colinfo / rowinfo)
+    alignas(16) uint32_t rowinfo_lo[RES_H];
+    alignas(16) uint32_t bgcol[RES_W];        // pad == 1: source column of the background image sampled by pixel column px, BG_NONE outside it
     uint32_t bgrow[RES_H];                    // pad == 1: atlas offset of the background row sampled by pixel row py, BG_NONE outside the image
-    uint32_t tjob_src[MAX_TILE_JOBS];         // tile copies to stage: texel offset in the table,
-    uint16_t tjob_dst[MAX_TILE_JOBS], tjob_words[MAX_TILE_JOBS];  // arena word offset, words
+    TileJob tjob[MAX_TILE_JOBS];              // tile copies to stage
     uint16_t cellmap[MAX_CELLS_1D * MAX_CELLS_1D];  // [ci * ny + cj], x outer / y inner = draw order
     alignas(16) Blit bg[MAX_BG_BLITS];
 
@@ -1248,7 +1255,6 @@ struct Raster {
             f.n_gen = 0;
             f.tile_top = 0;
             f.n_tjobs = 0;
-            f.n_strip_cols = 0;
             f.tile_w0 = f.tile_h0 = w0;
             f.cell_w = cw[2];
             f.rot = reinterpret_cast<RotBlit *>(c.rot_scratch_raw);
@@ -1310,12 +1316,15 @@ struct Raster {
         for (int j = ny + tid; j < Frame::kSpanBytes; j += nthreads) f.row_p1[j] = f.row_p2[j] = 255;
     }
 
-    // cell columns (rows) covering pixel column (row) p -> lo / hi and the packed CI_* word
+    // cell columns (rows) covering pixel column (row) p -> lo / hi and the packed CI_* words of hi and of lo
     // Spans are monotonic in the cell index (columns left to right; rows bottom-up, i.e. decreasing), so the
     // cells covering pixel p are a contiguous index range that two counts give: how many spans start at or
     // before p, how many end at or before p. Four spans per compare (byte-wise SIMD on the device).
+    static PG_HD uint32_t ci_word(const uint8_t *p1, const uint8_t *tsize, const uint8_t *k0, int base_mul, int px, int i) {
+        return (uint32_t)(i * base_mul) | CI_VALID | ((uint32_t)((px - p1[i] + k0[i]) & 31) << CI_D_SHIFT) | ((uint32_t)tsize[i] << CI_TW_SHIFT);
+    }
     static PG_HD uint32_t cell_lookup(const uint8_t *p1, const uint8_t *p2, const uint8_t *tsize, const uint8_t *k0, int n, int base_mul, int px, uint8_t &lo,
-                                      uint8_t &hi) {
+                                      uint8_t &hi, uint32_t &lo_word) {
         int started = 0, ended = 0;
 #if defined(__CUDA_ARCH__)
         const uint32_t pv = (uint32_t)px * 0x01010101u;
@@ -1344,12 +1353,16 @@ struct Raster {
         if (l > hgh) {
             lo = 255;
             hi = 0;
+            lo_word = 0;
             return 0;
         }
         lo = (uint8_t)l;
         hi = (uint8_t)hgh;
-        uint32_t w = (uint32_t)(hgh * base_mul) | CI_VALID | ((uint32_t)((px - p1[hgh] + k0[hgh]) & 31) << CI_D_SHIFT) | ((uint32_t)tsize[hgh] << CI_TW_SHIFT);
+        uint32_t w = ci_word(p1, tsize, k0, base_mul, px, hgh);
         w |= l != hgh ? CI_MULTI : CI_FAST;
+        if (hgh - l > 1)
+            w |= CI_WIDE;
+        lo_word = l == hgh ? w : ci_word(p1, tsize, k0, base_mul, px, l);
         return w;
     }
 
@@ -1625,31 +1638,27 @@ struct Raster {
     // ---- setup kernel, step 3: pixel -> cell lookups and the first pass over the visible cells
     static PG_HD void frame_build(Ctx &c, Frame &f, int tid, int nthreads, int /*unused*/) {
         const int wtid = tid, wn = nthreads;
-        if (f.pad == 1) {
+        {
             const Blit &b = f.bg[0];
-            for (int py = wtid; py < RES_H; py += wn) {
-                const uint32_t dy = (uint32_t)py - b.y1;
-                f.bgrow[py] = dy < b.h ? b.src + ((b.srcy + (uint32_t)b.iy * dy) >> 16) * b.sw : BG_NONE;
+            const bool one = f.pad == 1;
+            for (int p = wtid; p < RES_W + RES_H; p += wn) {
+                if (p < RES_W) {
+                    const uint32_t dx = (uint32_t)p - b.x1;
+                    f.bgcol[p] = one && dx < b.w ? (b.basex + (uint32_t)b.ix * dx) >> 16 : BG_NONE;
+                } else {
+                    const uint32_t dy = (uint32_t)(p - RES_W) - b.y1;
+                    f.bgrow[p - RES_W] = one && dy < b.h ? b.src + ((b.srcy + (uint32_t)b.iy * dy) >> 16) * b.sw : BG_NONE;
+                }
             }
         }
         if (!G::DRAWS_GRID)
             return;
         for (int px = wtid; px < RES_W + RES_H; px += wn) {
-            if (px < RES_W) {
-                const uint32_t w = cell_lookup(f.col_p1, f.col_p2, f.col_tw, f.col_k0, f.nx, f.ny, px, f.col_lo[px], f.col_hi[px]);
-                f.colinfo[px] = w;
-                if (w & CI_MULTI) {
-                    int slot;
-#if defined(__CUDA_ARCH__)
-                    slot = atomicAdd(&f.n_strip_cols, 1);
-#else
-                    slot = f.n_strip_cols++;
-#endif
-                    f.strip_cols[slot] = (uint8_t)px;
-                }
-            } else {
-                f.rowinfo[px - RES_W] = cell_lookup(f.row_p1, f.row_p2, f.row_th, f.row_k0, f.ny, 1, px - RES_W, f.row_lo[px - RES_W], f.row_hi[px - RES_W]);
-            }
+            if (px < RES_W)
+                f.colinfo[px] = cell_lookup(f.col_p1, f.col_p2, f.col_tw, f.col_k0, f.nx, f.ny, px, f.col_lo[px], f.col_hi[px], f.colinfo_lo[px]);
+            else
+                f.rowinfo[px - RES_W] = cell_lookup(f.row_p1, f.row_p2, f.row_th, f.row_k0, f.ny, 1, px - RES_W, f.row_lo[px - RES_W], f.row_hi[px - RES_W],
+                                                    f.rowinfo_lo[px - RES_W]);
         }
         // Cells, pass A (draw_grid_obj / draw_image for a grid cell, basic-abstract-game.cpp:877-919,
         // 940-950): a cell whose sprite can come from the pre-scaled tile table only registers the
@@ -1755,9 +1764,9 @@ struct Raster {
                     job = f.n_tjobs++;
 #endif
                     if (job < MAX_TILE_JOBS) {
-                        f.tjob_src[job] = tt.index[(slot * MAX_TILE_DIM + (tw - 1)) * MAX_TILE_DIM + (th - 1)];
-                        f.tjob_dst[job] = (uint16_t)off;
-                        f.tjob_words[job] = (uint16_t)words;
+                        f.tjob[job].src = tt.index[(slot * MAX_TILE_DIM + (tw - 1)) * MAX_TILE_DIM + (th - 1)];
+                        f.tjob[job].dst = (uint16_t)off;
+                        f.tjob[job].words = (uint16_t)words;
                         code = (uint16_t)(2 + off);
                     }
                 }
@@ -1846,6 +1855,14 @@ struct Raster {
 #endif
     }
 
+    static PG_HD int ctz32(uint32_t m) {  // m != 0
+#if defined(__CUDA_ARCH__)
+        return __ffs((int)m) - 1;
+#else
+        return __builtin_ctz(m);
+#endif
+    }
+
     // ---- phase D: composition. Colours are 0xFFRRGGBB (Format_RGB32).
     //   gather   per pixel: the grid cells over the background (draw_background + the cell loop of
     //            draw_foreground, basic-abstract-game.cpp:921-1007) — the cell under a pixel is a table
@@ -1863,12 +1880,6 @@ struct Raster {
         return f.arena[(int)code - 1 + dy * f.col_tw[ci] + dx];
     }
 
-    // pad == 1: source column of the background image for pixel column px (BG_NONE outside), and the texel
-    static PG_HD uint32_t bg_column(const Frame &f, int px) {
-        const Blit &b = f.bg[0];
-        const uint32_t dx = (uint32_t)px - b.x1;
-        return dx < b.w ? (b.basex + (uint32_t)b.ix * dx) >> 16 : BG_NONE;
-    }
     static PG_HD uint32_t bg_single(uint32_t bgrow, uint32_t bgcol, const uint32_t *atlas) {
         return (bgrow != BG_NONE && bgcol != BG_NONE) ? atlas[bgrow + bgcol] : 0xff000000u;  // fillRect(rect, black), basic-abstract-game.cpp:980
     }
@@ -1876,13 +1887,13 @@ struct Raster {
     static PG_HD_NOINLINE uint32_t bg_generic(const Frame &f, int px, int py, const uint32_t *atlas) {
         uint32_t dst = 0xff000000u;
         if (f.pad == 1)
-            return bg_single(f.bgrow[py], bg_column(f, px), atlas);
+            return bg_single(f.bgrow[py], f.bgcol[px], atlas);
         for (int i = 0; i < f.n_bg; i++) dst = layer_over(dst, blit_texel(f.bg[i], px, py, atlas, f.rot));
         return dst;
     }
 
-    // all cells over `under` at one pixel, in draw order (x outer / y inner): pixels where neighbouring
-    // cells overlap (the strips) or a cell is a general blit
+    // all cells over `under` at one pixel, in draw order (x outer / y inner), found by their spans: the
+    // fallback for pixels more than two cell columns (rows) cover
     static PG_HD uint32_t cells_over(const Frame &f, int px, int py, const uint32_t *atlas, uint32_t under) {
         uint32_t dst = under;
         const int clo = f.col_lo[px], chi = f.col_hi[px], rlo = f.row_lo[py], rhi = f.row_hi[py];
@@ -1900,126 +1911,110 @@ struct Raster {
         return cells_over(f, px, py, atlas, under);
     }
 
-    // What a thread keeps for the four pixel columns of its quad while it walks down the rows.
-    struct QuadCtx {
-        uint32_t ci[4];                    // colinfo (flags)
-        uint32_t cbase[4];                 // cell column * ny
-        uint32_t tile_dx[4], tile_tw[4];   // column of the pixel inside its cell's tile, row stride of that tile
-        uint32_t bg_sx[4];                 // single-image background: source column per pixel column (BG_NONE outside)
-        bool bg_one;
-    };
-    static PG_HD void quad_begin(const Frame &f, int px0, QuadCtx &q) {
-        q.bg_one = f.pad == 1;
-        for (int k = 0; k < 4; k++) {
-            const uint32_t ci = G::DRAWS_GRID ? f.colinfo[px0 + k] : 0u;
-            q.ci[k] = ci;
-            q.cbase[k] = ci & CI_BASE_MASK;
-            q.tile_dx[k] = (ci >> CI_D_SHIFT) & 31u;
-            q.tile_tw[k] = (ci >> CI_TW_SHIFT) & 31u;
-            q.bg_sx[k] = q.bg_one ? bg_column(f, px0 + k) : 0u;
+    // source value at a pixel of the cell that column word `cw` and row word `rw` (CI_* words) point at
+    static PG_HD uint32_t cell_texel(const Frame &f, uint32_t cw, uint32_t rw, int px, int py, const uint32_t *atlas) {
+        const uint32_t code = f.cellmap[(cw & CI_BASE_MASK) + (rw & CI_BASE_MASK)];
+        if (code == 0)
+            return 0;
+        if (code & CELL_GENERAL) {
+            const Blit &gb = *f.gen_blit((int)(code & 0x7fffu));
+            if (gb.kind == BLIT_SOLID) {  // solid-colour cells (chaser's orbs, monochrome mode) are a box test
+                const uint32_t box = *reinterpret_cast<const uint32_t *>(&gb);
+                const uint32_t ddx = (uint32_t)px - (box & 0xffu), ddy = (uint32_t)py - ((box >> 8) & 0xffu);
+                return (ddx < ((box >> 16) & 0xffu) && ddy < (box >> 24)) ? gb.src : 0u;
+            }
+            return blit_texel(gb, px, py, atlas, f.rot);  // other kinds take the long way
         }
+        return f.arena[code - 1 + ((rw >> CI_D_SHIFT) & 31u) * ((cw >> CI_TW_SHIFT) & 31u) + ((cw >> CI_D_SHIFT) & 31u)];
+    }
+
+    // The pixels off the one-tile-cell path: a one-pixel overlap strip of two cell columns and / or rows
+    // (up to 2 x 2 cells, blended in draw order: column lo, hi outer, row lo, hi inner) or a cell that is
+    // a general blit. `ci` / `ri` are the pixel's column / row words.
+    static PG_HD uint32_t cells_odd(const Frame &f, uint32_t ci, uint32_t ri, int px, int py, const uint32_t *atlas, uint32_t under) {
+        if ((ci | ri) & CI_WIDE)
+            return cells_generic(f, px, py, atlas, under);
+        const uint32_t cl = (ci & CI_MULTI) ? f.colinfo_lo[px] : ci;
+        const uint32_t rl = (ri & CI_MULTI) ? f.rowinfo_lo[py] : ri;
+        uint32_t dst = under;
+        if (ci & CI_MULTI) {
+            if (ri & CI_MULTI)
+                dst = layer_over(dst, cell_texel(f, cl, rl, px, py, atlas));
+            dst = layer_over(dst, cell_texel(f, cl, ri, px, py, atlas));
+        }
+        if (ri & CI_MULTI)
+            dst = layer_over(dst, cell_texel(f, ci, rl, px, py, atlas));
+        return layer_over(dst, cell_texel(f, ci, ri, px, py, atlas));
     }
 
     enum GatherMode { GATHER_ALL = 0, GATHER_BG = 1, GATHER_CELLS = 2 };  // background + cells | background only | cells over what fb holds
 
-    // Four horizontally adjacent pixels of row py -> fb. The inline part covers the common pixel —
-    // at most one cell and that one from a pre-scaled tile: tile texel first, the background (or
-    // what is already in fb) only when the texel is not opaque. Pixels of overlap strips are left to
-    // gather_strips (GATHER_ALL stores a placeholder there, GATHER_CELLS leaves fb alone).
+    // Four horizontally adjacent pixels of row py -> fb. The common pixel — at most one cell and that one
+    // from a pre-scaled tile — is one cellmap and one arena load; the four pixels then fetch what lies
+    // under them (the background, or what fb holds) in one pass, only where the texel is not opaque.
+    // Strip pixels and general-blit cells (`odd`) get cells_odd over that afterwards. `bgc` = the
+    // background source columns of the four pixels (pad == 1).
     template <int MODE>
-    static PG_HD void gather_quad(const Frame &f, const QuadCtx &q, int px0, int py, const uint32_t *atlas, uint32_t *fb) {
-        const uint32_t rowinfo = (G::DRAWS_GRID && MODE != GATHER_BG) ? f.rowinfo[py] : 0u;
-        const uint32_t bgrow = q.bg_one ? f.bgrow[py] : BG_NONE;
-        const uint32_t rbase = rowinfo & CI_BASE_MASK, dy = (rowinfo >> CI_D_SHIFT) & 31u;
+    static PG_HD void gather_quad(const Frame &f, const uint32_t *bgc, bool bg_one, int px0, int py, const uint32_t *atlas, uint32_t *fb) {
+        constexpr bool kCells = G::DRAWS_GRID && MODE != GATHER_BG;
         uint32_t *dst = fb + py * RES_W + px0;
-        uint32_t s[4];
-        uint32_t slow = 0, strip = 0;
-        for (int k = 0; k < 4; k++) {
-            s[k] = 0;
-            if (G::DRAWS_GRID && MODE != GATHER_BG) {
-                const uint32_t both = q.ci[k] & rowinfo;
+        uint32_t ci[4] = {0u, 0u, 0u, 0u}, s[4] = {0u, 0u, 0u, 0u};
+        uint32_t odd = 0;
+        const uint32_t rowinfo = kCells ? f.rowinfo[py] : 0u;
+        if (kCells && (rowinfo & CI_VALID)) {  // a cell row covers the pixel row
+#if defined(__CUDA_ARCH__)
+            const uint4 cv = *reinterpret_cast<const uint4 *>(f.colinfo + px0);
+            ci[0] = cv.x; ci[1] = cv.y; ci[2] = cv.z; ci[3] = cv.w;
+#else
+            for (int k = 0; k < 4; k++) ci[k] = f.colinfo[px0 + k];
+#endif
+            const uint32_t rbase = rowinfo & CI_BASE_MASK, dy = (rowinfo >> CI_D_SHIFT) & 31u;
+            for (int k = 0; k < 4; k++) {
+                const uint32_t both = ci[k] & rowinfo;
                 if (both & CI_FAST) {  // one cell column and one cell row cover the pixel
-                    const uint32_t code = f.cellmap[q.cbase[k] + rbase];
+                    const uint32_t code = f.cellmap[(ci[k] & CI_BASE_MASK) + rbase];
                     if (code & CELL_GENERAL) {
-                        // solid-colour cells (chaser's orbs, monochrome mode) are a box test; other kinds take the long way
+                        // solid-colour cells (half of chaser's pixels) are a box test; other kinds are odd
                         const Blit &gb = *f.gen_blit((int)(code & 0x7fffu));
                         if (gb.kind == BLIT_SOLID) {
                             const uint32_t box = *reinterpret_cast<const uint32_t *>(&gb);
                             const uint32_t ddx = (uint32_t)(px0 + k) - (box & 0xffu), ddy = (uint32_t)py - ((box >> 8) & 0xffu);
                             s[k] = (ddx < ((box >> 16) & 0xffu) && ddy < (box >> 24)) ? gb.src : 0u;
                         } else {
-                            slow |= 1u << k;
+                            odd |= 1u << k;
                         }
-                    } else if (code) {
-                        s[k] = f.arena[code - 1 + dy * q.tile_tw[k] + q.tile_dx[k]];
-                    }
+                    } else if (code)
+                        s[k] = f.arena[code - 1 + dy * ((ci[k] >> CI_TW_SHIFT) & 31u) + ((ci[k] >> CI_D_SHIFT) & 31u)];
                 } else if (both & CI_VALID) {
-                    strip |= 1u << k;
+                    odd |= 1u << k;
                 }
             }
         }
+        const uint32_t bgrow = bg_one ? f.bgrow[py] : BG_NONE;
         uint32_t c[4];
         for (int k = 0; k < 4; k++) {
             c[k] = s[k];
-            if ((strip >> k) & 1u)
-                continue;
-            if (s[k] >= 0xff000000u && !((slow >> k) & 1u))
-                continue;
+            if (s[k] >= 0xff000000u)
+                continue;  // opaque tile texel (odd pixels have s = 0)
             uint32_t under;
             if (MODE == GATHER_CELLS)
                 under = dst[k];
-            else if (q.bg_one)
-                under = bg_single(bgrow, q.bg_sx[k], atlas);
+            else if (bg_one)
+                under = bg_single(bgrow, bgc[k], atlas);
             else
                 under = bg_generic(f, px0 + k, py, atlas);
-            if ((slow >> k) & 1u)
-                c[k] = cells_generic(f, px0 + k, py, atlas, under);
-            else
-                c[k] = s[k] != 0 ? s[k] + pg_byte_mul(under, (~s[k]) >> 24) : under;
+            c[k] = s[k] != 0 ? s[k] + pg_byte_mul(under, (~s[k]) >> 24) : under;  // odd pixels: under
         }
-        if (MODE == GATHER_CELLS) {
-            for (int k = 0; k < 4; k++)
-                if (!((strip >> k) & 1u))
-                    dst[k] = c[k];
-        } else {
 #if defined(__CUDA_ARCH__)
-            *reinterpret_cast<uint4 *>(dst) = make_uint4(c[0], c[1], c[2], c[3]);
+        *reinterpret_cast<uint4 *>(dst) = make_uint4(c[0], c[1], c[2], c[3]);
 #else
-            for (int k = 0; k < 4; k++) dst[k] = c[k];
+        for (int k = 0; k < 4; k++) dst[k] = c[k];
 #endif
-        }
-    }
-
-    // The pixels gather_quad skipped: where neighbouring cell columns (rows) overlap by a pixel, up
-    // to 2 x 2 cells lie over each other. Those strips are a few pixel columns and rows of the frame;
-    // walked here densely (a lane = one strip pixel) they cost a fraction of what they cost as
-    // divergent branches of the quad loop.
-    template <int MODE>
-    static PG_HD void gather_strips(const Frame &f, uint32_t *fb, int row_first, int row_step, int lane, int nlanes, const uint32_t *atlas) {
-        const int my_rows = (RES_H - row_first + row_step - 1) / row_step;
-        // strip columns x my rows
-        const int n1 = f.n_strip_cols * my_rows;
-        for (int idx = lane; idx < n1; idx += nlanes) {
-            const int px = f.strip_cols[idx / my_rows], py = row_first + (idx % my_rows) * row_step;
-            if (!(f.rowinfo[py] & CI_VALID))
-                continue;  // no cell row here: gather_quad drew the pixel
-            uint32_t *dst = fb + py * RES_W + px;
-            const uint32_t under = MODE == GATHER_CELLS ? *dst : bg_generic(f, px, py, atlas);
-            *dst = cells_over(f, px, py, atlas, under);
-        }
-        // strip rows among my rows x the other columns
-        for (int r = 0; r < my_rows; r++) {
-            const int py = row_first + r * row_step;
-            if (!(f.rowinfo[py] & CI_MULTI))
-                continue;
-            for (int px = lane; px < RES_W; px += nlanes) {
-                const uint32_t ci = f.colinfo[px];
-                if (!(ci & CI_VALID) || (ci & CI_MULTI))
-                    continue;
-                uint32_t *dst = fb + py * RES_W + px;
-                const uint32_t under = MODE == GATHER_CELLS ? *dst : bg_generic(f, px, py, atlas);
-                *dst = cells_over(f, px, py, atlas, under);
-            }
+        // the odd pixels' cells over what was just stored there (one copy of that code, not four)
+        while (kCells && odd != 0) {
+            const int k = ctz32(odd);
+            odd &= odd - 1;
+            dst[k] = cells_odd(f, f.colinfo[px0 + k], rowinfo, px0 + k, py, atlas, dst[k]);
         }
     }
 
@@ -2080,41 +2075,55 @@ struct Raster {
 
     // Everything the owner of rows row_first, row_first + row_step, ... does to them: `lane` of
     // `nlanes` threads (a warp on the device; 16 quad columns x 2 interleaved row sets per lane pair)
-    static PG_HD void compose_rows(const Frame &f, uint32_t *fb, int row_first, int row_step, int lane, int nlanes, const uint32_t *atlas) {
-        const int nb = f.n_ent_below, n_all = f.n_ent + f.n_overlay;
+    template <int MODE>
+    static PG_HD void gather_rows(const Frame &f, uint32_t *fb, int row_first, int row_step, int lane, int nlanes, const uint32_t *atlas) {
         // lanes tile the rows: quad column = lane % 16, and lane / 16 picks every (nlanes / 16)-th of our rows
         const int per_row = RES_W / 4;
         const int sub = nlanes >= per_row ? nlanes / per_row : 1;
+        const bool bg_one = f.pad == 1;
         for (int qx = lane % per_row; qx < per_row; qx += (nlanes < per_row ? nlanes : per_row)) {
-            QuadCtx q;
-            quad_begin(f, qx * 4, q);
+            uint32_t bgc[4];
+            for (int k = 0; k < 4; k++) bgc[k] = f.bgcol[qx * 4 + k];
             const int first = row_first + row_step * (nlanes >= per_row ? lane / per_row : 0);
-            if (G::ENTS_BELOW_GRID && nb > 0) {
-                for (int py = first; py < RES_H; py += row_step * sub) gather_quad<GATHER_BG>(f, q, qx * 4, py, atlas, fb);
-            } else {
-                for (int py = first; py < RES_H; py += row_step * sub) gather_quad<GATHER_ALL>(f, q, qx * 4, py, atlas, fb);
-            }
+            for (int py = first; py < RES_H; py += row_step * sub) gather_quad<MODE>(f, bgc, bg_one, qx * 4, py, atlas, fb);
         }
-        if (G::DRAWS_GRID && !(G::ENTS_BELOW_GRID && nb > 0))
-            gather_strips<GATHER_ALL>(f, fb, row_first, row_step, lane, nlanes, atlas);
+    }
+    // `dbg` (profiling variant, PG_PHASE_TIMING): the first row owner's SM cycles in gather ([0]) and paint ([1])
+    static PG_HD void compose_rows(const Frame &f, uint32_t *fb, int row_first, int row_step, int lane, int nlanes, const uint32_t *atlas,
+                                   uint32_t *dbg = nullptr) {
+        const int nb = f.n_ent_below, n_all = f.n_ent + f.n_overlay;
+#if defined(PG_PHASE_TIMING) && defined(__CUDA_ARCH__)
+        const long long t0 = clock64();
+#endif
         if (G::ENTS_BELOW_GRID && nb > 0) {
+            gather_rows<GATHER_BG>(f, fb, row_first, row_step, lane, nlanes, atlas);
 #if defined(__CUDA_ARCH__)
             __syncwarp();
 #endif
             paint_blits(f, fb, 0, nb, row_first, row_step, lane, nlanes, atlas);
-            for (int qx = lane % per_row; qx < per_row; qx += (nlanes < per_row ? nlanes : per_row)) {
-                QuadCtx q;
-                quad_begin(f, qx * 4, q);
-                const int first = row_first + row_step * (nlanes >= per_row ? lane / per_row : 0);
-                for (int py = first; py < RES_H; py += row_step * sub) gather_quad<GATHER_CELLS>(f, q, qx * 4, py, atlas, fb);
-            }
-            if (G::DRAWS_GRID)
-                gather_strips<GATHER_CELLS>(f, fb, row_first, row_step, lane, nlanes, atlas);
+#if defined(__CUDA_ARCH__)
+            __syncwarp();
+#endif
+            gather_rows<GATHER_CELLS>(f, fb, row_first, row_step, lane, nlanes, atlas);
+        } else {
+            gather_rows<GATHER_ALL>(f, fb, row_first, row_step, lane, nlanes, atlas);
         }
 #if defined(__CUDA_ARCH__)
         __syncwarp();
 #endif
+#if defined(PG_PHASE_TIMING) && defined(__CUDA_ARCH__)
+        const long long t1 = clock64();
+#endif
         paint_blits(f, fb, (G::ENTS_BELOW_GRID ? nb : 0), n_all, row_first, row_step, lane, nlanes, atlas);
+#if defined(PG_PHASE_TIMING) && defined(__CUDA_ARCH__)
+        __syncwarp();
+        if (dbg && row_first == 0 && lane == 0) {
+            dbg[0] = (uint32_t)(t1 - t0);
+            dbg[1] = (uint32_t)(clock64() - t1);
+        }
+#else
+        (void)dbg;
+#endif
     }
 };
 

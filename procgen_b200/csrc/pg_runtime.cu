@@ -1075,6 +1075,16 @@ int pgb200_debug_phase_offset(void) {
 #endif
 }
 
+int pgb200_debug_pixel_classes(libenv_env *handle, int env, uint8_t *out) {
+    VecEnv *v = (VecEnv *)handle;
+    if (env < 0 || env >= v->num_envs)
+        return -1;
+    v->set_device();
+    v->sync();
+    const size_t gi = (size_t)env % v->games.size();
+    return v->games[gi]->pixel_classes[v->view[gi]](v->base, env, out);
+}
+
 int pgb200_consumer_slot(libenv_env *handle) { return ((VecEnv *)handle)->base.consumer_slot; }
 
 int pgb200_mirror_parity(libenv_env *handle) { return ((VecEnv *)handle)->mirror_parity; }

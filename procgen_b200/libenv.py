@@ -49,7 +49,8 @@ EXPORTS = ["libenv_version", "libenv_make", "libenv_get_tensortypes", "libenv_se
            "pgb200_sync", "pgb200_get_errors", "pgb200_debug_cycles", "pgb200_debug_read_env", "pgb200_kernel_launches", "pgb200_is_device_build",
            "pgb200_kernel_timing_begin", "pgb200_kernel_timing_end", "get_state", "set_state", "pgb200_set_launch_shape",
            "pgb200_frame_info", "pgb200_set_rgb_mirror", "pgb200_mirror_parity",
-           "pgb200_set_consumer_output", "pgb200_consumer_slot", "pgb200_debug_phase_offset"]
+           "pgb200_set_consumer_output", "pgb200_consumer_slot", "pgb200_debug_phase_offset",
+           "pgb200_debug_pixel_classes"]
 
 _lib = None
 

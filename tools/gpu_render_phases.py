@@ -27,9 +27,12 @@ for e in range(0, n, max(1, n // 512)):
     env._lib.pgb200_debug_read_env(env._h, int(e), buf, None, 0)
     acc.append(struct.unpack_from("<12I", bytes(buf), off))
 a = np.array(acc, dtype=np.float64)
-names = ["begin", "build(ents|cells A)", "jobs(tile alloc)", "stage+cells B", "tile wait", "compose", "consumer+pack", "store"]
-tot = a[:, :8].sum(1).mean()
+# render_kernel's phase counters (thread 0 of the CTA; ids 1-4 belong to the logic kernel's reset phases):
+# 0 stage (bulk copies of the frame record and tiles), 5 compose, 6 consumer + pack, 7 store; compose split
+# as warp 0 (row owner 0) sees it: 8 gather (cells over background), 9 paint (entity + overlay blits)
+phases = [(0, "stage"), (5, "compose"), (8, "  gather (warp 0)"), (9, "  paint (warp 0)"), (6, "consumer+pack"), (7, "store")]
+tot = a[:, [0, 5, 6, 7]].sum(1).mean()
 print(f"{game} {mode}: mean cycles per frame {tot:.0f}")
-for i, nm in enumerate(names):
+for i, nm in phases:
     print(f"  {nm:22s} mean {a[:, i].mean():8.0f}  p90 {np.percentile(a[:, i], 90):8.0f}  {100 * a[:, i].mean() / tot:5.1f}%")
 env.close()
